@@ -151,9 +151,10 @@ def synth_wav(rank: int, idx: int, B: int = HUBERT_B, S: int = HUBERT_S) -> torc
     return (0.1 * torch.randn(B, S, generator=g)).clamp_(-1, 1)
 
 
-def run_hubert_gpu(args, rank, local_rank, world, lib, dist):
+def run_hubert_gpu(args, rank, local_rank, world, lib, dist, outputs=None):
     """Secondary headline: HuBERT-25Hz unit extraction throughput (audio-hours/s), mHuBERT geometry, synthetic audio,
-    seeded random weights; every rank extracts its own batches (no collective on this path)."""
+    seeded random weights; every rank extracts its own batches (no collective on this path).  `outputs` (a dict, if
+    given) receives the unit ids and frame counts of the last timed batch."""
     import ctypes as C
     from slamkit_b200.feature_extractor import HubertB200Config, HubertB200FeatureExtractor, random_params
     dev = torch.device("cuda", local_rank)
@@ -162,7 +163,7 @@ def run_hubert_gpu(args, rank, local_rank, world, lib, dist):
                                     max_samples=HUBERT_S)
     host = [synth_wav(rank, i).pin_memory() for i in range(2)]
     devw = [h.to(dev) for h in host]
-    n = max(50, args.steps)                              # SURVEY.md §8d: >= 50 timed batches
+    n = args.steps
 
     def sync():
         if world > 1:
@@ -183,11 +184,13 @@ def run_hubert_gpu(args, rank, local_rank, world, lib, dist):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for i in range(n):
-        fe.units_device(devw[i % 2], None)
+        last = fe.units_device(devw[i % 2], None)
     e1.record()
     sync()
     dev_ms = mx(e0.elapsed_time(e1))
     launches = lib.sk_launch_count() - l0
+    if outputs is not None:
+        outputs["hubert_units"], outputs["hubert_frames"] = (t.cpu() for t in last)
     def e2e_plain():
         for i in range(n):
             ids, nf = fe.units_device(host[i % 2], None)       # pinned host -> device inside, on the compute stream
@@ -239,11 +242,11 @@ def run_hubert_gpu(args, rank, local_rank, world, lib, dist):
     sync()
     r0, r1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     r0.record()
-    for i in range(10):
+    for i in range(n):
         fe.units_device(ragged, lens_d)
     r1.record()
     sync()
-    ragged_ms = mx(r0.elapsed_time(r1)) / 10
+    ragged_ms = mx(r0.elapsed_time(r1)) / n
 
     ids_h, e2e_ms = timed(e2e_plain)
     e2e_mode = "H2D on the compute stream"
@@ -319,7 +322,40 @@ CFG4_VOCAB = 151_665 + 502      # Qwen2.5 tokenizer entries + 500 units + <speec
 CFG4_TOKENS = 8192              # packed tokens per GPU and step: documents of <= 2048 tokens in ONE row (DataCollatorWithFlattening)
 
 
+DUMP_SAMPLE = 1 << 20          # elements kept of each parameter-sized buffer by --dump-outputs
+DUMP_LIMIT = 64 << 20
+
+
+def lm_step_outputs(model, opt, returned) -> dict:
+    """What a caller of a train step holds once it returns: the step's return values, the loss statistics of its last
+    forward pass, the optimiser's clip statistics, and the same seeded sample of the updated parameters, the step's
+    gradients and the AdamW moments (each full buffer holds one bf16 value per parameter, 0.7 GB for the default
+    workload).  Copied to the host, so later work cannot change it."""
+    g = torch.Generator().manual_seed(0)
+    idx = torch.randint(0, model.n_params, (min(DUMP_SAMPLE, model.n_params),), generator=g).sort().values
+    idx_d = idx.to(model.device)
+    out = {**returned, "lm_stats": model.stats, "optimizer_stats": opt.stats, "sample_index": idx,
+           "params_sample": model.params[idx_d], "grads_sample": model.grads[idx_d],
+           "exp_avg_sample": opt.exp_avg[idx_d], "exp_avg_sq_sample": opt.exp_avg_sq[idx_d]}
+    return {k: torch.as_tensor(v).detach().cpu() for k, v in out.items()}
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """One DIR/<name>.npy per array: integers as float64 (exact), floating point (bf16 / fp32) as float32 (exact)."""
+    import numpy as np
+    conv = {}
+    for name, t in arrays.items():
+        t = torch.as_tensor(t).detach().cpu()
+        conv[name] = (t.double() if (t.dtype == torch.float64 or not t.is_floating_point()) else t.float()).numpy()
+    total = sum(a.nbytes for a in conv.values())
+    assert total <= DUMP_LIMIT, f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT} byte budget"
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in conv.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def _timed_steps(step, n_warm, n_steps, dist, world, dev):
+    """Returns (device ms, wall ms) of the n_steps timed steps and what the last of them returned."""
     def barrier():
         if world > 1:
             dist.barrier()
@@ -327,11 +363,12 @@ def _timed_steps(step, n_warm, n_steps, dist, world, dev):
     for i in range(n_warm):
         step(i)
     barrier()
+    last = None
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     t0 = time.perf_counter()
     e0.record()
     for i in range(n_steps):
-        step(i)
+        last = step(i)
     e1.record()
     barrier()
     ms = max(e0.elapsed_time(e1), 0.0)
@@ -340,7 +377,7 @@ def _timed_steps(step, n_warm, n_steps, dist, world, dev):
         t = torch.tensor([ms, wall], device=dev, dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms, wall = float(t[0]), float(t[1])
-    return ms, wall
+    return ms, wall, last
 
 
 def run_cfg4(args, rank, local_rank, world, lib, dist):
@@ -370,14 +407,16 @@ def run_cfg4(args, rank, local_rank, world, lib, dist):
                          "n_items": n_lab, "n_tokens": n_lab}, lens))
     devb = [{k: (v.to(dev) if torch.is_tensor(v) else v) for k, v in b.items()} for b, _ in batches]
     l0 = lib.sk_launch_count()
-    ms, _ = _timed_steps(lambda i: trainer.train_step([devb[i % 2]]), max(args.warmup, 3), args.steps, dist, world, dev)
+    ms, _, last = _timed_steps(lambda i: trainer.train_step([devb[i % 2]]), max(args.warmup, 3), args.steps, dist, world, dev)
     launches = lib.sk_launch_count() - l0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, lm_step_outputs(model, trainer.opt, {"loss": last}))
 
     def e2e(i):
         b = {k: (v.to(dev, non_blocking=True) if torch.is_tensor(v) else v) for k, v in batches[i % 2][0].items()}
         trainer.train_step([b])
         return trainer.last_loss()
-    ms2, wall2 = _timed_steps(e2e, 2, args.steps, dist, world, dev)
+    ms2, wall2, _ = _timed_steps(e2e, 2, args.steps, dist, world, dev)
     if rank == 0:
         n_mm = 24 * 14_909_440 + CFG4_VOCAB * 896
         attn = sum(3 * 24 * 4 * n * n * 896 // 2 for n in batches[0][1])      # causal, per document
@@ -427,8 +466,10 @@ def run_cfg5(args, rank, local_rank, world, lib, dist):
         host.append((ids.pin_memory(), labels.pin_memory()))
     devb = [(a.to(dev), b.to(dev)) for a, b in host]
     l0 = lib.sk_launch_count()
-    ms, _ = _timed_steps(lambda i: tr.step(*devb[i % 2]), max(args.warmup, 3), args.steps, dist, world, dev)
+    ms, _, last = _timed_steps(lambda i: tr.step(*devb[i % 2]), max(args.warmup, 3), args.steps, dist, world, dev)
     launches = lib.sk_launch_count() - l0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, lm_step_outputs(pol, tr.opt, last))
     loss_host = torch.zeros((), dtype=torch.float32).pin_memory()
 
     def e2e(i):
@@ -436,7 +477,7 @@ def run_cfg5(args, rank, local_rank, world, lib, dist):
         out = tr.step(a.to(dev, non_blocking=True), b.to(dev, non_blocking=True))
         loss_host.copy_(out["loss"], non_blocking=False)
         return float(loss_host)
-    ms2, wall2 = _timed_steps(e2e, 2, args.steps, dist, world, dev)
+    ms2, wall2, _ = _timed_steps(e2e, 2, args.steps, dist, world, dev)
     if rank == 0:
         tok = 16 * SEQ
         flop = (2 * 2 + 6) * N_MATMUL_PARAMS * tok + (2 + 3) * 24 * (4 * SEQ * 896) // 2 * tok   # ref fwd + policy fwd/bwd
@@ -473,6 +514,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--skip-hubert", action="store_true", help="skip the secondary HuBERT audio-hours/s measurement")
     ap.add_argument("--hubert-cpu", action="store_true", help=argparse.SUPPRESS)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last of them computed (rank 0) as DIR/<name>.npy: returned "
+                         "loss, loss / clip statistics, a seeded sample of the parameters, gradients and AdamW moments, and "
+                         "the HuBERT leg's unit ids; the inputs are the same on every run")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
@@ -516,7 +561,7 @@ def main():
         counts.update({"n_items_global": PER_GPU_BATCH * SEQ * world, "n_tokens_global": PER_GPU_BATCH * SEQ * world})
 
     def step_device(i):
-        trainer.train_step([{"input_ids": devb[i % NB], "labels": devb[i % NB], **counts}])
+        return trainer.train_step([{"input_ids": devb[i % NB], "labels": devb[i % NB], **counts}])
 
     def step_e2e(i):
         # host ids in (one pinned-host -> device copy feeds input_ids and labels: a causal LM's labels ARE its ids),
@@ -548,11 +593,12 @@ def main():
     barrier()
     e0.record()
     for i in range(args.steps):
-        step_device(i)
+        last = step_device(i)
     e1.record()
     barrier()
     dev_ms = max_over_ranks(e0.elapsed_time(e1))
     launches = lib.sk_launch_count() - launches0
+    outputs = lm_step_outputs(model, trainer.opt, {"loss": last}) if args.dump_outputs and rank == 0 else None
 
     # end-to-end through the public API with host buffers
     for i in range(2):
@@ -631,7 +677,7 @@ def main():
     if not args.skip_hubert:
         del devb
         try:
-            hubert = run_hubert_gpu(args, rank, local_rank, world, lib, dist)
+            hubert = run_hubert_gpu(args, rank, local_rank, world, lib, dist, outputs)
         except Exception as e:      # the secondary leg must never cost the primary line
             hubert = {"metric": "HuBERT-25Hz unit extraction audio-hours/sec", "value": None,
                       "error": f"{type(e).__name__}: {e}"}
@@ -655,6 +701,8 @@ def main():
                         "d2h_bytes_per_step": 4, "ms_per_step": e2e_ms / args.steps},
                 "gpu_launches": int(launches), "roofline": roof, "cpu_baseline": cpu, "final_loss": loss,
                 "secondary": hubert}
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

@@ -16,6 +16,12 @@ What is pinned:
   lm_loglik.npz    reference `UnitLM.log_likelihood` (sum and mean forms) on a right-padded batch, seeded weights.
   hubert_tiny.npz  reference `HubertFeatureExtractor.extract` + `batch_cluster` (HF HubertModel, sklearn
                    KMeans.predict) on seeded weights: small mHuBERT-25Hz-geometry model, 2 ragged clips.
+  lm_checkpoint.npz  what the reference's `UnitLM.from_pretrained` makes of a directory written by
+                   `slamkit_b200.lm.write_unit_lm_checkpoint` (seed-3 weights): its state-dict names and shapes, the
+                   architecture it resolves from config.json, and its bf16 logits on seeded ids.
+  audio{1,2}_head.flac  the first FLAC_HEAD_FRAMES frames of the reference's example_data/audio/audio{1,2}.flac, byte for
+                   byte (libFLAC-encoded LPC streams), with the padding block dropped and STREAMINFO's sample count and
+                   MD5 set to those of the kept frames; needs the built library (the decoder checks the full files first).
 """
 import json
 import os
@@ -260,13 +266,107 @@ def make_hubert_golden(out_path: str):
     print("hubert golden ->", out_path, "frames", hs.shape, "lens", [len(t) for t in toks])
 
 
+def make_checkpoint_golden(out_path: str):
+    """The reference's `UnitLM.from_pretrained` on a checkpoint directory our writer produced."""
+    import safetensors.torch
+    from transformers import OPTConfig
+    import slamkit.model.unit_lm as ref_mod
+    from oracle.lm_oracle import OracleLMConfig, forward_logits, init_params
+    from slamkit_b200.lm import LMConfig, write_unit_lm_checkpoint
+    ocfg = OracleLMConfig(vocab_size=502, hidden=128, n_layers=2, n_heads=2, n_kv_heads=1, head_dim=64, ffn=256)
+    p = init_params(ocfg, seed=3)
+    tmp = tempfile.mkdtemp()
+    base, ck = os.path.join(tmp, "base"), os.path.join(tmp, "ck")
+    os.makedirs(base)
+    write_unit_lm_checkpoint(ck, p, LMConfig(vocab_size=502, hidden=128, n_layers=2, n_heads=2, n_kv_heads=1, head_dim=64,
+                                             ffn=256), base_model_name=base)
+    json.dump(json.load(open(os.path.join(ck, "config.json")))["base_config"], open(os.path.join(base, "config.json"), "w"))
+    # HF builds a default UnitLMConfig() to diff configs, whose base model is looked up on the hub (unit_lm.py:37,66-70)
+    real = ref_mod.AutoConfig.from_pretrained
+    ref_mod.AutoConfig.from_pretrained = lambda name, *a, **k: OPTConfig() if name == "facebook/opt-350M" else real(name, *a, **k)
+    try:
+        model = ref_mod.UnitLM.from_pretrained(ck, torch_dtype=torch.bfloat16)
+    finally:
+        ref_mod.AutoConfig.from_pretrained = real
+    sd = model.state_dict()
+    assert all(torch.equal(sd[k], p[k]) for k in p)
+    assert set(safetensors.torch.load_file(os.path.join(ck, "model.safetensors"))) <= set(sd)
+    g = torch.Generator().manual_seed(1)
+    ids = torch.randint(2, 502, (2, 24), generator=g)
+    ids[:, 0] = 1
+    with torch.no_grad():
+        logits = model(input_ids=ids).logits.to(torch.bfloat16)
+        assert torch.equal(logits, forward_logits(p, ocfg, ids).to(torch.bfloat16))
+    z = np.load(os.path.join(ROOT, "tests", "golden", "lm_loglik.npz"))
+    ll = model.log_likelihood(torch.from_numpy(z["tokens"]), mean_nll=False)
+    assert np.allclose(ll.float().numpy(), z["ll_sum"], rtol=1e-5, atol=1e-4)
+    lc = model.lm.config
+    arch = {"model_type": lc.model_type, "hidden_size": lc.hidden_size, "intermediate_size": lc.intermediate_size,
+            "num_hidden_layers": lc.num_hidden_layers, "num_attention_heads": lc.num_attention_heads,
+            "num_key_value_heads": lc.num_key_value_heads, "vocab_size": lc.vocab_size, "rms_norm_eps": lc.rms_norm_eps,
+            "tie_word_embeddings": lc.tie_word_embeddings, "rope_theta": lc.rope_parameters["rope_theta"],
+            "pad_token_id": model.config.base_config.pad_token_id}
+    names = sorted(sd)
+    np.savez_compressed(out_path, ids=ids.numpy(), logits_u16=bf16_to_u16(logits), names=np.array(names),
+                        shapes=np.array([json.dumps(list(sd[k].shape)) for k in names]), arch=np.array(json.dumps(arch)))
+    print("checkpoint golden ->", out_path, arch)
+
+
+FLAC_HEAD_FRAMES = 8
+
+
+def make_flac_head_golden(src: str, out_path: str, n_frames: int = FLAC_HEAD_FRAMES):
+    import hashlib
+    from slamkit_b200.audio_io import flac_decode_int, flac_info
+
+    def crc8(b):
+        c = 0
+        for x in b:
+            c ^= x
+            for _ in range(8):
+                c = ((c << 1) ^ 0x07) & 0xff if c & 0x80 else (c << 1) & 0xff
+        return c
+
+    info = flac_info(src)
+    pcm = flac_decode_int(src)
+    assert hashlib.md5(pcm.astype("<i2").tobytes()).digest() == info["md5"]      # the full decode is the encoder's audio
+    d = open(src, "rb").read()
+    assert d[:4] == b"fLaC"
+    pos, blocks, last = 4, [], False
+    while not last:
+        last, kind, n = d[pos] & 0x80, d[pos] & 0x7f, int.from_bytes(d[pos + 1:pos + 4], "big")
+        if kind != 1:                                                               # drop PADDING
+            blocks.append(bytearray(d[pos:pos + 4 + n]))
+        pos += 4 + n
+    bs = int.from_bytes(blocks[0][4 + 2:4 + 4], "big")                              # fixed block size (max = min)
+    assert blocks[0][0] & 0x7f == 0 and bs == int.from_bytes(blocks[0][4:6], "big") and bs == 4096
+    # frame n_frames starts at the first sync code whose header (coded frame number, CRC-8) says so
+    end = pos
+    while True:
+        end = d.index(b"\xff\xf8", end + 1)
+        if d[end + 2:end + 4] == d[pos + 2:pos + 4] and d[end + 4] == n_frames and crc8(d[end:end + 5]) == d[end + 5]:
+            break
+    n = n_frames * bs
+    si = blocks[0]
+    si[4 + 13] = (si[4 + 13] & 0xf0) | ((n >> 32) & 0xf)
+    si[4 + 14:4 + 18] = (n & 0xffffffff).to_bytes(4, "big")
+    si[4 + 18:4 + 34] = hashlib.md5(pcm[:n].astype("<i2").tobytes()).digest()
+    for b in blocks:
+        b[0] &= 0x7f
+    blocks[-1][0] |= 0x80
+    open(out_path, "wb").write(b"fLaC" + b"".join(blocks) + d[pos:end])
+    got = flac_decode_int(out_path)
+    assert flac_info(out_path)["num_frames"] == n and np.array_equal(got, pcm[:n])
+    print("flac head golden ->", out_path, n, "samples", os.path.getsize(out_path), "bytes")
+
+
 if __name__ == "__main__":
     assert os.path.isdir(REF), "the reference is only mounted in the build container"
     _stub_omegaconf()
     sys.path.insert(0, REF)
     gd = os.path.join(ROOT, "tests", "golden")
     os.makedirs(gd, exist_ok=True)
-    which = sys.argv[1:] or ["lm", "packed", "loglik", "tokeniser", "hubert"]
+    which = sys.argv[1:] or ["lm", "packed", "loglik", "tokeniser", "hubert", "checkpoint", "flac"]
     if "loglik" in which:
         make_loglik_golden(os.path.join(gd, "lm_loglik.npz"))
     if "lm" in which:
@@ -277,3 +377,9 @@ if __name__ == "__main__":
         make_tokeniser_golden(os.path.join(gd, "tokeniser.npz"))
     if "hubert" in which:
         make_hubert_golden(os.path.join(gd, "hubert_tiny.npz"))
+    if "checkpoint" in which:
+        make_checkpoint_golden(os.path.join(gd, "lm_checkpoint.npz"))
+    if "flac" in which:
+        for name in ("audio1", "audio2"):
+            make_flac_head_golden(os.path.join(REF, "example_data", "audio", f"{name}.flac"),
+                                  os.path.join(gd, f"{name}_head.flac"))

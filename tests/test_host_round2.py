@@ -14,7 +14,6 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLDEN = os.path.join(ROOT, "tests", "golden")
-REF = "/root/reference"
 
 
 # ------------------------------------------------------------------------------------------------ GradSync
@@ -189,46 +188,45 @@ def test_checkpoint_layout_round_trip(tmp_path):
     assert c["base_config"]["num_key_value_heads"] == 1 and c["vocab_size"] == 502 and c["twist_init"] is False
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="the reference checkout exists only in the build container")
-def test_reference_unit_lm_loads_a_b200_checkpoint(tmp_path, monkeypatch):
-    """SURVEY.md §8 f-4: the reference's own `UnitLM.from_pretrained` consumes the directory `save_pretrained` writes, and
-    its logits / log_likelihood on it equal the oracle's (which the GPU path is tested against)."""
+def test_reference_unit_lm_loads_a_b200_checkpoint(tmp_path):
+    """SURVEY.md §8 f-4: the reference's own `UnitLM.from_pretrained` consumes the directory `save_pretrained` writes.
+    tests/golden/lm_checkpoint.npz holds what it made of such a directory (oracle/make_goldens.py): the parameter names
+    and shapes it loaded, the architecture it read from config.json, and its logits.  The directory written now must
+    give the same names, shapes and architecture, and the model it describes (run by the oracle) the reference's logits
+    and, under the reference's log_likelihood rule (unit_lm.py:184-194, calc_nll), its tests/golden/lm_loglik.npz."""
+    from helpers import u16_to_bf16
     from oracle import lm_oracle as O
+    from safetensors.torch import load_file
     from slamkit_b200.lm import write_unit_lm_checkpoint
-    m = types.ModuleType("omegaconf")
-    m.DictConfig, m.ListConfig, m.OmegaConf = type("DictConfig", (dict,), {}), type("ListConfig", (list,), {}), type("OmegaConf", (), {})
-    sys.modules.setdefault("omegaconf", m)
-    if REF not in sys.path:
-        sys.path.insert(0, REF)
-    import slamkit.model.unit_lm as ref_mod
-    from slamkit.model.unit_lm import UnitLM
-    from transformers import OPTConfig
-    # HF builds a default-constructed UnitLMConfig() to diff configs, and the reference's default base model is looked up
-    # on the hub (unit_lm.py:37,66-70): stand in for that one lookup, everything else is the reference's own code path
-    real = ref_mod.AutoConfig.from_pretrained
-    monkeypatch.setattr(ref_mod.AutoConfig, "from_pretrained",
-                        staticmethod(lambda name, *a, **k: OPTConfig() if name == "facebook/opt-350M" else real(name, *a, **k)))
-    ocfg = O.OracleLMConfig(vocab_size=502, hidden=128, n_layers=2, n_heads=2, n_kv_heads=1, head_dim=64, ffn=256)
-    p = O.init_params(ocfg, seed=3)
-    base = tmp_path / "base"
-    os.makedirs(base)
-    ck = tmp_path / "ck"
-    write_unit_lm_checkpoint(str(ck), p, _tiny_cfg(), base_model_name=str(base))
-    json.dump(json.load(open(ck / "config.json"))["base_config"], open(base / "config.json", "w"))   # offline stand-in for the hub
-    model = UnitLM.from_pretrained(str(ck), torch_dtype=torch.bfloat16)
-    sd = model.state_dict()
+    p = O.init_params(O.OracleLMConfig(vocab_size=502, hidden=128, n_layers=2, n_heads=2, n_kv_heads=1, head_dim=64,
+                                       ffn=256), seed=3)
+    write_unit_lm_checkpoint(str(tmp_path), p, _tiny_cfg(), base_model_name="Qwen/Qwen2.5-0.5B")
+    z = np.load(os.path.join(GOLDEN, "lm_checkpoint.npz"))
+    ref_shapes = {str(k): tuple(json.loads(str(s))) for k, s in zip(z["names"], z["shapes"])}
+    sd = load_file(str(tmp_path / "model.safetensors"))
+    assert {k: tuple(v.shape) for k, v in sd.items()} == {k: s for k, s in ref_shapes.items() if k != "lm.lm_head.weight"}
+    assert "lm.lm_head.weight" in ref_shapes                                       # the reference ties it to the embedding
     assert all(torch.equal(sd[k], p[k]) for k in p), [k for k in p if not torch.equal(sd[k], p[k])][:3]
-    g = torch.Generator().manual_seed(1)
-    ids = torch.randint(2, 502, (2, 24), generator=g)
-    ids[:, 0] = 1
+    base = json.load(open(tmp_path / "config.json"))["base_config"]
+    arch = json.loads(str(z["arch"]))
+    assert {k: base[k] for k in arch} == arch
+    assert base["tie_word_embeddings"] and base["hidden_size"] // base["num_attention_heads"] == 64
+    ocfg = O.OracleLMConfig(vocab_size=base["vocab_size"], hidden=base["hidden_size"], n_layers=base["num_hidden_layers"],
+                            n_heads=base["num_attention_heads"], n_kv_heads=base["num_key_value_heads"], head_dim=64,
+                            ffn=base["intermediate_size"], rms_eps=base["rms_norm_eps"], rope_theta=base["rope_theta"])
     with torch.no_grad():
-        ref_logits = model(input_ids=ids).logits
+        logits = O.forward_logits(sd, ocfg, torch.from_numpy(z["ids"]))
+    assert torch.equal(logits.to(torch.bfloat16), u16_to_bf16(z["logits_u16"]))
+    zl = np.load(os.path.join(GOLDEN, "lm_loglik.npz"))
+    tokens = torch.from_numpy(zl["tokens"])
     with torch.no_grad():
-        logits = O.forward_logits(p, ocfg, ids)
-    assert torch.equal(ref_logits.to(torch.bfloat16), logits.to(torch.bfloat16))
-    z = np.load(os.path.join(GOLDEN, "lm_loglik.npz"))
-    ll = model.log_likelihood(torch.from_numpy(z["tokens"]), mean_nll=False)
-    assert np.allclose(ll.float().numpy(), z["ll_sum"], rtol=1e-5, atol=1e-4)
+        logits = O.forward_logits(sd, ocfg, tokens)
+    target = tokens[:, 1:].clone()
+    target[target == base["pad_token_id"]] = -100
+    nll = torch.nn.functional.cross_entropy(logits[:, :-1].reshape(-1, logits.shape[-1]), target.reshape(-1),
+                                            reduction="none").view(target.shape)
+    ll = -(nll * target.ne(-100)).sum(-1)
+    assert np.allclose(ll.float().numpy(), zl["ll_sum"], rtol=1e-5, atol=1e-4)
 
 
 def test_checkpoint_rotation_and_listing(tmp_path):
